@@ -10,15 +10,20 @@ A *step* is one mini-batch of ``--batch`` samples on EVERY worker (weak scaling:
 including that worker's share of the parameter-server traffic (one fused commit + pull every
 ``--window`` steps).  The timed quantity is a *region* of exactly ``--steps`` = K consecutive steps:
 
-* ``value``  device-timed, max over ranks.  Every region is ONE CUDA graph of K training steps with the
+* ``value``  device-timed, max over ranks.  A region is ONE CUDA graph of K training steps with the
              algorithm's exchanges at the iterations where they fall (K need not be a multiple of the
-             window: the graphs cycle through the window phases).  After >= W warm-up steps that replay
-             every graph once, R >= 50 regions run back to back, each bracketed by CUDA events on the
-             worker's stream; ``ms_per_step * steps`` is the MEAN region time of the slowest rank, so
-             every timed step is in steady state and every rank performs R*K/window exchanges.
+             window: the warm-up graphs cycle through the window phases).  After >= W warm-up steps that
+             replay every graph once, one region of exactly K steps, starting at a window boundary, is
+             bracketed by CUDA events on the worker's stream; ``ms_per_step * steps`` is the region time of
+             the slowest rank.  Larger K gives a steadier number.
 * ``e2e``    the same metric through the public API (``ADAG(...).train(dataset)``): every step's
              inputs are DMA'd from pinned host memory (uint8 pixels + int32 label) and every step's
              loss / accuracy record is read back to the host; timed on the device per graph replay.
+
+``--dump-outputs DIR`` writes what the timed region computed, as float32 ``.npy`` files (rank 0): ``center``
+(the parameter-server model a trainer returns), ``weights`` (the worker replica) and ``loss_accuracy`` (one
+row per timed step; the last row is the last step).  Inputs and initial weights are seeded, so two builds
+can be compared output for output with the same arguments.
 
 ``--impl reference`` runs the UNMODIFIED reference (``baseline/_ref``) on shimmed Keras / Spark
 substrates for the same model / trainer / window / batch (``baseline/reference_arm.py``).
@@ -142,6 +147,33 @@ class ClockSampler:
                 "samples": len(sm), "window": window, "reasons": sorted(reasons)}
 
 
+DUMP_BYTES = 64 * 2**20
+
+
+def dump_outputs(out_dir: str, region, shard_regions, shards, worker, steps: int, parity: int) -> None:
+    """Write what the timed region computed (see ``--dump-outputs``).  Call after the device synchronise
+    that ends the region.  An array larger than its share of DUMP_BYTES is replaced by a fixed, seeded
+    sample of its elements (same indices in every run with the same arguments)."""
+    import numpy as np
+
+    if shards:
+        by_ptr = {r.center_ptr: r for r in shard_regions}
+        center = np.concatenate([by_ptr[ptr].read_center()[:hi - lo].numpy() for lo, hi, ptr in shards])
+    else:
+        center = region.read_center().numpy()
+    outs = {"center": center,
+            "weights": worker.rep.W.detach().float().cpu().numpy(),
+            "loss_accuracy": worker.hist_host[parity][:steps].numpy().copy()}
+    share = DUMP_BYTES // len(outs)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outs.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.nbytes > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def auto_steps_per_graph(tau: int, batch: int) -> int:
     """Mirror of FabricWorker's default: ~8k rows per graph replay, whole windows."""
     return max(1, min(64, -(-8192 // (tau * batch)))) * tau
@@ -224,13 +256,16 @@ def main() -> None:
     ap.add_argument("--comm", default="default", choices=["default", "exchange", "commit_pull", "fused_pull"])
     ap.add_argument("--dedicated-ps", action="store_true", help="rank 0 hosts the center only (N-1 workers)")
     ap.add_argument("--sharded-ps", action="store_true", help="slice r of the center lives in rank r's HBM")
-    ap.add_argument("--reps", type=int, default=0, help="timed K-step regions (0 = auto: >= 50, ~1 s)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed region's outputs (center, worker weights, per-step loss / accuracy) as .npy")
     ap.add_argument("--no-fuse-comm", action="store_true",
                     help="A/B: window-boundary exchange as separate kernels instead of inside the backward-update kernel")
     ap.add_argument("--skip-e2e", action="store_true")
     ap.add_argument("--backend", default="fabric", choices=["fabric", "nccl"],
                     help="nccl = the library-only baseline trainer (autograd replicas + all-reduce), e2e only")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "native" or args.backend != "fabric" or args.dedicated_ps):
+        ap.error("--dump-outputs needs the native fabric arm with a worker on rank 0 (no --dedicated-ps)")
 
     if args.impl == "reference":
         reference_arm(args)
@@ -355,18 +390,13 @@ def main() -> None:
                     e1.record(worker.compute)
                     events.append((e0, e1))
 
+        # a whole number of periods: the timed region starts at a window boundary on staging parity 0
         warm_regions = max(period, -(-W // K))
         warm_regions += (-warm_regions) % period
         with torch.cuda.stream(worker.compute):
-            cal = []
-            run_regions(0, warm_regions, cal)
+            run_regions(0, warm_regions)
         torch.cuda.synchronize()
-        cal_ms = statistics.median(a.elapsed_time(b) for a, b in cal)
-        R = args.reps if args.reps > 0 else int(min(4000, max(50, 1000.0 / max(cal_ms, 1e-3))))
-        R += (-R) % period
-    else:
-        R = 0
-    R = max(gather(R))        # every rank times the same number of regions
+    R = 1                     # one timed region: exactly K timed steps
     if is_worker:
         worker.launched = worker.exchanges = 0
         barrier()
@@ -376,6 +406,8 @@ def main() -> None:
             run_regions(warm_regions, R, events)
         torch.cuda.synchronize()
         sampler.mark_end()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, region, shard_regions, shards, worker, K, warm_regions & 1)
         barrier()
         rep_ms = [a.elapsed_time(b) for a, b in events]
         # the exchange alone, all ranks at once (PS ingress / egress contention included)

@@ -378,8 +378,12 @@ def test_single_worker_center_matches_hand_replay(rule, cls, kw, hp):
 @pytest.mark.parametrize("cls,kw", [(ADAG, dict(communication_window=4)),
                                     (AEASGD, dict(communication_window=4, rho=1.0, learning_rate=0.1)),
                                     (EAMSGD, dict(communication_window=4, rho=0.1, learning_rate=1.0, momentum=0.5))])
-def test_library_collectives_baseline_backend(cls, kw):
+def test_library_collectives_baseline_backend(cls, kw, monkeypatch):
     """backend="nccl" (gloo on a CPU host): two spawned ranks, bulk-synchronous all-reduce every window."""
+    # the CPU host path on any machine: on a GPU host the backend runs one rank per GPU, so a one-GPU host
+    # would train a single worker
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")       # the spawned ranks
+    monkeypatch.setattr(torch.cuda, "device_count", lambda: 0)   # the launcher (CUDA may be initialised here)
     ds = tiny_data(1024)
     t = cls(tiny_model(0), {"class_name": "adam", "config": {"lr": 0.02}}, "categorical_crossentropy", num_workers=2,
             batch_size=16, num_epoch=2, **kw)

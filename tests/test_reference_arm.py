@@ -32,6 +32,38 @@ def test_reference_arm_runs_the_unmodified_package():
     assert "distkeras_b200" not in src
 
 
+def test_adag_matches_recorded_reference_run():
+    """``tests/golden/reference_arm_adag_mnist_mlp.json`` is what ``bench.py --impl reference --steps 5 --warmup 3``
+    printed when the unmodified reference ran (CPU, one worker).  The same job through this package's ADAG must do
+    the same bookkeeping: W + K steps recorded per worker and the reference's update counter (starts at 1, one
+    increment per committed window)."""
+    import torch
+
+    import bench
+    from distkeras_b200 import trainers
+    from distkeras_b200.data import Dataset
+    from distkeras_b200.models import ZOO
+
+    rec = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_arm_adag_mnist_mlp.json")))
+    assert rec["impl"] == "reference" and rec["value"] > 0 and rec["unit"] == "samples/s"
+    cfg = rec["config"]
+    assert cfg["trainer"] == "ADAG" and cfg["batch_per_worker"] == bench.DEFAULT_BATCH[cfg["model"]] == 64
+    assert cfg["communication_window"] == bench.DEFAULT_WINDOW["adag"]
+    B, tau, steps = cfg["batch_per_worker"], cfg["communication_window"], rec["warmup"] + rec["steps"]
+    g = torch.Generator().manual_seed(0)
+    x = torch.rand(steps * B, *bench.IN_SHAPE[cfg["model"]], generator=g)
+    y = torch.randint(0, 10, (steps * B,), generator=g).to(torch.int32)
+    t = trainers.ADAG(ZOO[cfg["model"]](seed=0), cfg["worker_optimizer"], "categorical_crossentropy",
+                      num_workers=cfg["num_workers"], batch_size=B, communication_window=tau)
+    t.backend = "thread"
+    t.train(Dataset({"features": x, "label": y}))
+    per_worker = {}
+    for h in t.get_history():
+        per_worker[h["worker_id"]] = per_worker.get(h["worker_id"], 0) + 1
+    assert sorted(per_worker.values()) == rec["steps_done_per_worker"]
+    assert t.num_updates() == rec["num_updates"] == 1 + steps // tau
+
+
 def test_shims_live_outside_the_reference_package():
     shims = os.path.join(ROOT, "baseline", "shims")
     assert {"keras", "pyspark", "tensorflow"} <= set(os.listdir(shims))
